@@ -146,8 +146,8 @@ def _cpu_case(n_images):
 
 
 def reference_kind():
-    """'reference' when the unmodified reference can run here (staged into baseline/_ref by
-    tools/stage_reference.py, or /root/reference itself), else 'port' (the oracle)."""
+    """'reference' when the unmodified original project can run here (staged into oracle/_ref
+    by build() from the original checkout), else 'port' (the oracle)."""
     from oracle import reference_lift as RL
     return 'reference' if RL.available() else 'port'
 
@@ -250,12 +250,27 @@ def run_reference(args):
                          'sample': '%d image(s) of the batch per step (same geometry; images are '
                                    'independent, the rate is per ray), torch CPU fp32, no_grad; %s'
                                    % (n_img, 'unmodified reference render (run.py:176-350 lifted '
-                                      'from baseline/_ref), planes given' if kind == 'reference'
+                                      'from oracle/_ref), planes given' if kind == 'reference'
                                       else 'oracle port of the reference ops')},
         'e2e': {'value': value, 'unit': UNIT, 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0},
         'gpu_launches': 0,
     }
     print(json.dumps(line))
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes each [batch, ...] output as out_dir/<name>.npy in float32, so that two builds can be
+    compared output for output on the same seeded inputs.  Past DUMP_LIMIT_BYTES in all, only the
+    leading images of the batch are written (the same ones every run)."""
+    import numpy as np
+    per_image = sum(t[0].numel() for t in outputs.values()) * 4
+    keep = max(1, min(min(len(t) for t in outputs.values()), DUMP_LIMIT_BYTES // per_image))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t[:keep].detach().float().cpu().numpy())
 
 
 # ------------------------------------------------------------------ the B200 arm
@@ -412,6 +427,8 @@ class Bench:
         self.barrier()
         clocks = sampler.summary() if rank == 0 else None
         ms_step = self.max_over_ranks(ev0.elapsed_time(ev1)) / a.steps
+        if a.dump_outputs and rank == 0:
+            dump_outputs(a.dump_outputs, dict(zip(('rgb', 'depth', 'mask'), last)))
         rays_step = gb * H * W
         value = rays_step / (ms_step * 1e-3)
         k_ms = sum(x.elapsed_time(y) for x, y in kernel_events) / max(1, len(kernel_events))
@@ -635,7 +652,7 @@ class Bench:
         from nerf_from_image_b200.synthesis import FusedSynthesis
         from oracle import reference_lift as RL  # availability probe + module import only
         if not RL.available():
-            return {'unavailable': 'reference files not staged (tools/stage_reference.py)'}
+            return {'unavailable': 'original project not staged (oracle/_ref)'}
         try:
             import types
             dev = self.dev
@@ -777,7 +794,7 @@ class Bench:
         cpu = {'value': rate, 'unit': UNIT, 'cores': cores, 'host_cores': os.cpu_count(), 'kind': kind,
                'sample': '%d of the 32 images (same geometry) x %d passes, %.1f s, torch CPU fp32 '
                          'no_grad, %s' % (n_img, reps, dt, 'unmodified reference render lifted from '
-                                          'baseline/_ref' if kind == 'reference' else 'oracle port')}
+                                          'oracle/_ref' if kind == 'reference' else 'oracle port')}
         # parity of the CUDA path on exactly those images, against the oracle with the same
         # injected noise (the reference draws its own: same distribution, different numbers)
         from oracle import render_oracle as O
@@ -917,10 +934,17 @@ def main():
     ap.add_argument('--quick', action='store_true', help='skip the side legs (ncu, A/B runs)')
     ap.add_argument('--e2e-steps', type=int, default=3)
     ap.add_argument('--mlp-mode', type=lambda x: int(x, 0), default=0)
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='config 2: write rgb / depth / mask of the last timed step to '
+                         'DIR/<name>.npy (float32, at most 64 MB in all)')
     args = ap.parse_args()
     args.steps_given = args.steps is not None
     if args.steps is None:
         args.steps = 20 if args.impl == 'b200' else 3
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'b200' or args.config != 2):
+        ap.error('--dump-outputs writes the outputs of the timed render of --config 2')
     if args.impl == 'reference':
         return run_reference(args)
     args.warmup = max(args.warmup, 3)

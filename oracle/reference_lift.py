@@ -1,16 +1,15 @@
-"""Run the UNMODIFIED reference hot path -- TEST / BASELINE INFRASTRUCTURE.
+"""Run the UNMODIFIED original project's hot path -- TEST / BASELINE INFRASTRUCTURE.
 
-/root/reference is mounted read-only in the build container and does not exist
-on the GPU box; there the same files are found, unmodified, under the git-ignored
-``baseline/_ref/`` (staged by ``tools/stage_reference.py`` from ``__graft_entry__.build()``).
-Everything here is optional: ``available()`` says whether the reference can be
-imported; callers are ``tests/`` (oracle pinning, golden generation, the on-GPU
-``render()`` drop-in tests) and ``bench.py``'s reference legs (``--impl reference``,
-``cpu_baseline``) -- never the product path.  No reference source is copied:
-``render`` (run.py:176-350) is taken from the reference file by AST at run
+The original project is optional: ``build()`` stages the files used here, unmodified, from its
+checkout into the git-ignored ``oracle/_ref/`` (``oracle/stage_reference.py``), and
+``available()`` says whether they can be imported.  Callers
+are the golden-data generators under ``tests/golden/``, the on-GPU drop-in tests that need the
+original ``Generator`` module, and ``bench.py``'s reference legs (``--impl reference``,
+``cpu_baseline``) -- never the product path.  No original source is copied into the
+repository: ``render`` (run.py:176-350) is taken from the original file by AST at run
 time (run.py itself cannot be imported -- it parses argv, loads datasets and
 imports lpips/pytorch_fid at module level), and the radiance field is the
-reference's own ``models.generator.Generator`` whose synthesis network is
+original's own ``models.generator.Generator`` whose synthesis network is
 swapped for a stub that returns the planes under test.
 """
 
@@ -23,15 +22,16 @@ import warnings
 import torch
 import torch.nn.functional as F
 
-_STAGED = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))),
-                       'baseline', '_ref')
+_STAGED = os.path.join(os.path.dirname(os.path.abspath(__file__)), '_ref')
 
 
 def _find_root():
-    for cand in (os.environ.get('NFI_REFERENCE_ROOT'), '/root/reference', _STAGED):
+    """NFI_REFERENCE_ROOT, else the copy build() staged, else the original checkout itself."""
+    from oracle.stage_reference import DEFAULT_SOURCE
+    for cand in (os.environ.get('NFI_REFERENCE_ROOT'), _STAGED, DEFAULT_SOURCE):
         if cand and os.path.isfile(os.path.join(cand, 'run.py')):
             return cand
-    return '/root/reference'
+    return _STAGED
 
 
 REFERENCE_ROOT = _find_root()

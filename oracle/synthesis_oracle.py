@@ -7,8 +7,8 @@ sm_100a kernels of ``nerf_from_image_b200/csrc/nfi_synth.cu`` (SURVEY.md section
 Only ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py``'s reference legs import it.
 
 Pinned to the reference: ``tests/test_synthesis_oracle.py`` runs the UNMODIFIED
-``models.stylegan.SynthesisNetwork`` (imported from /root/reference or the staged
-``baseline/_ref``) on the same weights and latents and compares every block; the fixtures under
+``models.stylegan.SynthesisNetwork`` (imported from the staged
+``oracle/_ref``) on the same weights and latents and compares every block; the fixtures under
 ``tests/golden/synth/`` were produced by the reference (``tests/golden/make_golden_synth.py``).
 
 Per layer (models/stylegan.py:114-145 ``conv_modulated2d``, :293-356 ``SynthesisLayer``):

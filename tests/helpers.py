@@ -1,8 +1,22 @@
 """Shared helpers for the parity tests (oracle side and CUDA side)."""
+import os
+
+import numpy as np
 import torch
 
 from fixtures import synthetic
 from oracle import render_oracle as O
+
+REFERENCE_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'reference')
+
+
+def reference_golden(test, key):
+    """{output name: tensor} the original project returned for parameter set ``key`` of
+    ``test`` (recorded by tests/golden/make_golden_reference.py)."""
+    z = np.load(os.path.join(REFERENCE_GOLDEN, test + '.npz'))
+    out = {k[len(key) + 1:]: torch.from_numpy(z[k]) for k in z.files if k.startswith(key + '/')}
+    assert out, 'no stored reference outputs for %s / %s' % (test, key)
+    return out
 
 CASES = {
     # name: (dataset, camera kwargs, scene kwargs)

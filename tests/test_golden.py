@@ -2,7 +2,7 @@
 
 CPU: the oracle reproduces every fixture (forward and reference-autograd
 gradients) -- this is what pins the oracle to the reference on a machine that
-has no /root/reference.  GPU: the CUDA path reproduces them through the C ABI.
+has no checkout of the original project.  GPU: the CUDA path reproduces them through the C ABI.
 """
 import glob
 import os

@@ -43,15 +43,22 @@ def test_white_background_only_adds_one_minus_mask():
 
 def test_images_are_independent():
     """No cross-image arithmetic (SURVEY.md section 8e): any permutation or subset of the batch
-    renders to the same pixels -- the premise of sharding by image."""
+    renders to the same pixels -- the premise of sharding by image.  Both renders run on one CPU
+    thread: with 16 or more, ATen splits the oracle's work by position in the batch, and the last
+    bit of a pixel can then depend on where its image sits."""
     scene, cams, nt, nu = case()
-    full = Hh.run_oracle(scene, cams, H, W, S, nt, nu)
-    perm = torch.tensor([2, 0, 1])
-    per_image = ('planes', 'palette', 'c2w', 'focal', 'center', 'bbox')
-    sel = lambda d: {k: (v[perm] if (k in per_image and v is not None) else v)
-                     for k, v in d.items()}
-    out = Hh.run_oracle(sel(scene), sel(cams), H, W, S, nt[perm],
-                        nu.view(3, H * W, S)[perm].reshape(-1, S))
+    threads = torch.get_num_threads()
+    torch.set_num_threads(1)
+    try:
+        full = Hh.run_oracle(scene, cams, H, W, S, nt, nu)
+        perm = torch.tensor([2, 0, 1])
+        per_image = ('planes', 'palette', 'c2w', 'focal', 'center', 'bbox')
+        sel = lambda d: {k: (v[perm] if (k in per_image and v is not None) else v)
+                         for k, v in d.items()}
+        out = Hh.run_oracle(sel(scene), sel(cams), H, W, S, nt[perm],
+                            nu.view(3, H * W, S)[perm].reshape(-1, S))
+    finally:
+        torch.set_num_threads(threads)
     for k in ('rgb', 'depth', 'mask'):
         assert torch.equal(out[k], full[k][perm]), k
 

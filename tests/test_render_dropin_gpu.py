@@ -3,9 +3,9 @@
 seeded) on CUDA, against the UNMODIFIED reference ``render`` (run.py:176-350, lifted by AST)
 running eagerly in fp32 on the same GPU from the same seed.
 
-/root/reference does not exist on the GPU box: the reference files are staged, unmodified,
-into the git-ignored ``baseline/_ref/`` by ``tools/stage_reference.py`` (run from
-``__graft_entry__.build()``); without them these tests skip and say so.
+The original project's files are staged, unmodified, into the git-ignored ``oracle/_ref/`` by
+``__graft_entry__.build()`` when NFI_REFERENCE_ROOT names a checkout of it; without them these
+tests skip and say so.
 
 What this pins that the CPU seam test (tests/test_render_dropin.py, CUDA core stood in for
 by the oracle) cannot: closure introspection on CUDA tensors, the no-copy plane join, the
@@ -21,7 +21,7 @@ from oracle import reference_lift as RL
 
 pytestmark = [pytest.mark.gpu,
               pytest.mark.skipif(not RL.available(),
-                                 reason='reference files not staged (tools/stage_reference.py)')]
+                                 reason='original project not staged (oracle/_ref)')]
 
 H = W = 32
 S = 16

@@ -1,6 +1,6 @@
 """The sm_100a tri-plane producer (csrc/nfi_synth.cu through nfi_synthesis_forward) against
 (1) the fixtures the reference produced, (2) the oracle restatement on a seeded mid-size
-network, and (3) -- where the reference files are staged (baseline/_ref) -- the UNMODIFIED
+network, and (3) -- where the original project is staged (oracle/_ref) -- the UNMODIFIED
 models.stylegan.SynthesisNetwork at the real size (256^2 planes, 512 channels), including RNG
 consumption of the noise draws.  Bar: <= 1e-3 relative L2 (BASELINE north_star); 3xTF32 leaves
 about 1e-6, the asserts use 5e-5."""
@@ -53,7 +53,7 @@ def test_against_the_oracle(cuda_lib, channels, batch):
 
 
 staged = pytest.mark.skipif(not RL.available(),
-                            reason='reference files not staged (tools/stage_reference.py)')
+                            reason='original project not staged (oracle/_ref)')
 
 
 @staged

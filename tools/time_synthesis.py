@@ -12,7 +12,7 @@ torch.backends.cudnn.allow_tf32 = False
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 32
 K = int(sys.argv[2]) if len(sys.argv) > 2 else 5
 if not RL.available():
-    raise SystemExit('reference files not staged (tools/stage_reference.py)')
+    raise SystemExit('original project not staged (oracle/_ref)')
 RL._import_reference()
 from models import stylegan
 torch.manual_seed(1234)
